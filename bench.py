@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (our arm: sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K ...  (reference arm: the CPU path on host cores)
+    python bench.py ... --dump-outputs DIR                   (also write the last timed step's embeddings as DIR/*.npy)
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on at one GPU):
     ONE-PEACE 4B vision-branch forward — `extract_image_features` on 64 synthetic 224x224 images per GPU:
@@ -91,6 +92,15 @@ def peaks():
         p = json.load(open(path))
         return p, "measured (MEASURED_PEAKS.json)"
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(out_dir, arrays, suffix=""):
+    """Write each tensor as float32 `out_dir/<name><suffix>.npy`, so that two builds run with the same arguments (hence the
+    same seeded weights and inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), t.detach().float().cpu().numpy())
 
 
 class ClockSampler:
@@ -205,7 +215,7 @@ def run_b200(args):
         l0 = K.LAUNCHES
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         clocks = sampler.stop() if sampler is not None else None
@@ -214,13 +224,17 @@ def run_b200(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, K.LAUNCHES - l0, clocks
+        return ms, K.LAUNCHES - l0, clocks, out
 
     warmup = max(3, args.warmup)
-    ms, launches, clocks = timed(step_core, args.steps, warmup, ClockSampler(local_rank) if rank == 0 else None)
+    ms, launches, clocks, core_out = timed(step_core, args.steps, warmup, ClockSampler(local_rank) if rank == 0 else None)
     value = BATCH * world * args.steps / (ms / 1e3)
-    ms_e2e, _, _ = timed(step_e2e, args.steps, warmup)
+    ms_e2e, _, _, e2e_out = timed(step_e2e, args.steps, warmup)
     e2e_value = BATCH * world * args.steps / (ms_e2e / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image_features": core_out, "e2e_image_features": e2e_out},
+                     "" if world == 1 else f"_rank{rank}")
+    del core_out, e2e_out
 
     # ---- per-kernel device times (CUDA events on the launching stream) for the roofline block ----
     roof = None
@@ -717,7 +731,7 @@ def run_reference(args):
     if rank != 0:
         return
     n = args.gpus
-    steps, warmup = max(1, min(args.steps, 2)), min(args.warmup, 1)
+    steps, warmup = args.steps, min(args.warmup, 1)
     r = cpu_reference(steps=steps, warmup=warmup, sample_images=8)
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": n, "steps": steps,
             "warmup": warmup, "ms_per_step": round(1e3 * r["seconds"] / steps, 1), "higher_is_better": True,
@@ -727,15 +741,28 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def _positive_int(s):
+    n = int(s)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {n}")
+    return n
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=_positive_int, default=20, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the contrastive / eager-baseline / hbm_kernels blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the image embeddings of the last timed step of the device path "
+                         "(image_features) and of the public-API path (e2e_image_features) as DIR/<name>.npy, float32 "
+                         "[64, 1536] each (names get _rank<r> with --gpus > 1)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the b200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:

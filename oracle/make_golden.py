@@ -90,8 +90,10 @@ def main():
         "outputs": dict(text=text, image=image, audio=audio),
         "adapter": dict(text_x=tx, text_pad=tpad, text_bias=tbias[0][0], image_x=ix[:1].clone(), image_bias=ibias[0][0, :, :40, :40].clone(),
                         audio_x=ax, audio_bias=abias[0][0]),
-        "text_layer0_out": l0,
     }, os.path.join(OUT, "tiny_retrieval.pt"))
+    # a file of its own keeps every golden file under 1 MB
+    torch.save({"config": cfgd, "weights_seed": 0, "inputs_seed": 0, "text_layer0_out": l0},
+               os.path.join(OUT, "tiny_text_layer0.pt"))
 
     # ---- gradients of the reference modules (torch autograd through the reference's own forward) ----
     # Summaries only (norm, seeded random projection, first 256 elements per parameter): they pin the oracle's

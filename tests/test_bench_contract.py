@@ -26,6 +26,21 @@ def test_reference_arm_prints_the_contract_line():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_reference_arm_runs_the_requested_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "3", "--warmup", "0"],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 3 and "x 3 step(s)" in d["cpu_baseline"]["sample"]
+
+
+def test_bad_arguments_are_refused():
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=300,
+                           cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, argv
+
+
 def test_product_arm_needs_cuda():
     if torch.cuda.is_available():
         return

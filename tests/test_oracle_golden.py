@@ -51,12 +51,14 @@ def test_audio_adapter(tiny):
     torch.testing.assert_close(bias, fx["adapter"]["audio_bias"], atol=0, rtol=0)
 
 
-def test_text_layer0(tiny):
+def test_text_layer0(tiny, golden_dir):
     fx, sd, cfg, (tok, _, _, _) = tiny
+    l0 = torch.load(os.path.join(golden_dir, "tiny_text_layer0.pt"), weights_only=False)
+    assert (l0["config"], l0["weights_seed"], l0["inputs_seed"]) == (fx["config"], fx["weights_seed"], fx["inputs_seed"])
     x, pad, bias = R.text_adapter(sd, cfg, tok)
     x = x * (1 - pad.unsqueeze(-1).type_as(x))
     y = R.encoder_layer(sd, cfg, x, bias, pad, "text", "encoder_wrapper.fusion_model.layers.0.")
-    torch.testing.assert_close(y, fx["text_layer0_out"], atol=2e-5, rtol=1e-5)
+    torch.testing.assert_close(y, l0["text_layer0_out"], atol=2e-5, rtol=1e-5)
 
 
 @pytest.mark.parametrize("modality", ["text", "image", "audio"])
